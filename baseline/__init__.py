@@ -1,1 +1,1 @@
-"""Harness around the UNMODIFIED reference (installed into baseline/_ref by install_ref.sh)."""
+"""Harness around the UNMODIFIED reference (copied into oracle/_ref by oracle/install_ref.sh)."""

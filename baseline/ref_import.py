@@ -1,9 +1,10 @@
 """Import the unmodified reference (zgcr/SimpleAICV_pytorch_training_examples).
 
-Search order: ``baseline/_ref`` (the offline pip install made by ``baseline/install_ref.sh``; it is
-git-ignored but travels to the GPU box with the gpurun snapshot), then ``/root/reference`` (build
-container only).  ``tools.utils`` / ``tools.scripts`` import ``calflops`` and ``pycocotools`` at module
-level (tools/utils.py:19, tools/scripts.py:14-15) which are not installed here; the hot path never
+The reference lives in ``oracle/_ref`` (git-ignored), copied there by ``oracle/install_ref.sh``.
+Only the golden-data generators under ``tests/golden`` and the torch baselines import it; the tests,
+``smoke()`` and ``bench.py`` compare with the stored golden data instead.  ``tools.utils`` /
+``tools.scripts`` import ``calflops`` and ``pycocotools`` at module level (tools/utils.py:19,
+tools/scripts.py:14-15), which are not installed here; the hot path never
 calls them, so empty stub modules are registered for those two names only.
 
 TEST / BENCH INFRASTRUCTURE: the product package never imports this module.
@@ -14,7 +15,7 @@ import sys
 import types
 
 _HERE = os.path.dirname(os.path.abspath(__file__))
-CANDIDATES = [os.path.join(_HERE, '_ref'), '/root/reference']
+CANDIDATES = [os.path.join(os.path.dirname(_HERE), 'oracle', '_ref')]
 
 
 def root():
@@ -31,7 +32,7 @@ def available():
 def _ensure_path():
     r = root()
     if r is None:
-        raise ImportError('reference not installed: run baseline/install_ref.sh in the build container')
+        raise ImportError('reference not installed: run oracle/install_ref.sh <reference checkout>')
     if r not in sys.path:
         sys.path.insert(0, r)
     for name in ('calflops', 'pycocotools', 'pycocotools.coco', 'pycocotools.cocoeval', 'pycocotools.mask'):

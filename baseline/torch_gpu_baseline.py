@@ -1,6 +1,6 @@
 """The target north_star names: the UNMODIFIED reference training loop under torch DDP on this box.
 
-Everything on the timed path is the reference's own code imported from baseline/_ref (install_ref.sh):
+Everything on the timed path is the reference's own code imported from oracle/_ref (oracle/install_ref.sh):
 ``backbones.__dict__[name]`` builds the model, ``tools.utils.set_seed / build_optimizer / Scheduler /
 build_training_mode`` (DistributedDataParallel + GradScaler) prepare it and ``tools.scripts.train_classification``
 runs the steps — host syncs, per-step barrier and all (tools/scripts.py:141-270).  Only the data is synthetic
@@ -129,7 +129,7 @@ def main():
     dist.all_reduce(ms, op=dist.ReduceOp.MAX)
     if rank == 0:
         amp = str(ref_scripts.get_amp_type(model))
-        line = {'what': 'unmodified reference (baseline/_ref) under torch DDP, its own train_classification loop',
+        line = {'what': 'unmodified reference (oracle/_ref) under torch DDP, its own train_classification loop',
                 'model': a.model, 'variant': a.variant, 'amp_type': amp, 'n_gpus': world, 'per_gpu_batch': a.batch,
                 'steps': a.steps, 'warmup': a.warmup, 'ms_per_step': float(ms), 'images_per_sec': a.batch * world / float(ms) * 1e3,
                 'wall_ms_per_step_rank0': wall / a.steps * 1e3, 'avg_loss': float(loss),

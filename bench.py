@@ -8,9 +8,10 @@ tools/scripts.py:141-270 in the reference.  The same JSON line carries a ``vit_b
 (BASELINE configs[2]: ViT-B/16, soft labels, AdamW with layer-wise lr decay) measured the same way.
 
   python bench.py [--gpus N] [--steps K] [--warmup W]     our arm (sm_100a kernels)
-  python bench.py --impl reference ...                    reference arm: the reference's CPU path (its own
-                                                          modules from baseline/_ref, else the oracle port)
-Prints ONE JSON line (rank 0).  See DESIGN.md "Measurement" for what every key means.
+  python bench.py --impl reference ...                    reference arm: the reference's step arithmetic on the
+                                                          host cores (the oracle port, fp32)
+  python bench.py ... --dump-outputs DIR                  also write what the last timed step computed as DIR/*.npy
+Every timed loop runs K steps.  Prints ONE JSON line (rank 0).  See DESIGN.md "Measurement" for what every key means.
 """
 import argparse
 import contextlib
@@ -25,6 +26,7 @@ import time
 ROOT = os.path.dirname(os.path.abspath(__file__))
 sys.path.insert(0, ROOT)
 
+import numpy as np  # noqa: E402
 import torch  # noqa: E402
 import torch.distributed as dist  # noqa: E402
 
@@ -149,48 +151,24 @@ def synthetic_batch(model_name, B, rank, pin):
 
 # --------------------------------------------------------------------------------------------
 def cpu_reference_step_times(model_name, batch, warmup, steps, threads):
-    """The reference's CPU path on this box's host cores: the UNMODIFIED reference modules (baseline/_ref;
-    model, criterion and tools.utils.build_optimizer) driven through the arithmetic of one
-    tools/scripts.py:141-270 step in fp32 (its entry points hard-require CUDA/NCCL, SURVEY.md 0.6).
-    Falls back to the oracle port when the reference install is absent.  Returns (kind, [seconds per step])."""
+    """The reference's CPU path on the host cores: the oracle port of the reference's model code (oracle/, pinned to
+    the reference by tests/golden) driven through the arithmetic of one tools/scripts.py:141-270 step in fp32 (its
+    entry points hard-require CUDA/NCCL, SURVEY.md 0.6).  Returns (kind, [seconds per step])."""
     torch.set_num_threads(threads)
     _retain_freed_host_memory()
     x, y = synthetic_batch(model_name, batch, 0, False)
-    from baseline import ref_import
-    if ref_import.available():
-        kind = 'reference'
-        backbones = ref_import.backbones()
-        ref_losses = ref_import.module('SimpleAICV.classification.losses')
-        ref_utils = ref_import.module('tools.utils')
-        torch.manual_seed(0)
+    kind = 'port'
+    from oracle import convnets, train_step, vit
+    sd = convnets.init_state('resnet50', 1000, 0) if model_name == 'resnet50' else vit.init_state(model_name, 1000, 0)
+    buf = {}
+
+    def step():
         if model_name == 'resnet50':
-            model, crit = backbones.resnet50(num_classes=1000), ref_losses.CELoss()
-            opt, _ = ref_utils.build_optimizer(r50_optimizer_cfg(), model)
+            _, loss, grads = train_step.loss_and_grads(sd, x, y, 'resnet50')
         else:
-            model = backbones.vit_base_patch16(image_size=224, num_classes=1000, drop_path_prob=0.1, global_pool=True)
-            crit = ref_losses.OneHotLabelCELoss()
-            opt, _ = ref_utils.build_optimizer(vit_optimizer_cfg(model), model)
-        model.train()
-
-        def step():
-            loss = crit(model(x), y)
-            loss.backward()
-            opt.step()
-            opt.zero_grad()
-            return loss.item()
-    else:
-        kind = 'port'
-        from oracle import convnets, train_step, vit
-        sd = convnets.init_state('resnet50', 1000, 0) if model_name == 'resnet50' else vit.init_state(model_name, 1000, 0)
-        buf = {}
-
-        def step():
-            if model_name == 'resnet50':
-                _, loss, grads = train_step.loss_and_grads(sd, x, y, 'resnet50')
-            else:
-                _, loss, grads = vit.loss_and_grads(sd, x, y, model_name, global_pool=True)
-            train_step.sgd_step(sd, grads, buf, 0.1)
-            return float(loss)
+            _, loss, grads = vit.loss_and_grads(sd, x, y, model_name, global_pool=True)
+        train_step.sgd_step(sd, grads, buf, 0.1)
+        return float(loss)
     times = []
     for i in range(warmup + steps):
         t0 = time.perf_counter()
@@ -232,7 +210,7 @@ def cpu_baseline_record(model_name, batch, warmup, steps):
     return {'value': batch / med, 'unit': 'images/s', 'cores': threads, 'kind': kind,
             'value_best': batch / best, 'sec_per_step_median': med, 'sec_per_step_min': best,
             'sample': (f'{steps} timed steps of batch {batch} after {warmup} warm-ups of the same {model_name} training step '
-                       f'(fwd+loss+bwd+optimizer), fp32, {"unmodified reference modules (baseline/_ref)" if kind == "reference" else "oracle port"}, '
+                       f'(fwd+loss+bwd+optimizer), fp32, oracle port, '
                        f'torch {torch.__version__} CPU, {threads} threads on {phys} physical cores; median reported'),
             'physical_cores': phys}
 
@@ -242,7 +220,7 @@ def run_reference(args, rank):
     if rank != 0:
         return
     batch = 16
-    warmup, steps = max(2, min(args.warmup, 3)), max(5, min(args.steps, 8))
+    warmup, steps = max(2, min(args.warmup, 3)), args.steps
     cb = cpu_baseline_record(args.model, batch, warmup, steps)
     line = {
         'impl': 'reference', 'metric': METRICS[args.model], 'value': cb['value'], 'unit': 'images/s', 'n_gpus': args.gpus, 'steps': steps,
@@ -518,11 +496,16 @@ def measure_model(model_name, args, rank, world, local_rank, dump_path=None, wit
     sampler = ClockSampler(local_rank)
     if rank == 0:
         sampler.start()
-    steps = args.steps if model_name != 'sam_h_encoder' else max(3, args.steps // 3)
+    steps = args.steps
     capturable_step = detr_masks is None     # DETRLoss matches on the host (a sync per step) and DETR trains with dropout
+    last = {}                                # the loss of the latest timed step, for --dump-outputs
+
+    def keep(fn):
+        return lambda: last.__setitem__('loss', fn())
+
     l0 = _lib.launch_count()
-    ms_total = timed(lambda: step(x_dev, y_dev), steps)
-    launches = (_lib.launch_count() - l0) * args.steps // steps
+    ms_total = timed(keep(lambda: step(x_dev, y_dev)), steps)
+    launches = _lib.launch_count() - l0
     eager_ms_step = ms_total / steps
 
     # end to end through the public API: every step's batch comes from pinned host memory through
@@ -555,13 +538,15 @@ def measure_model(model_name, args, rank, world, local_rank, dump_path=None, wit
     # device-resident throughput: the same graph replayed on resident inputs when there is one, else the eager loop above
     if split is not None:
         split([x_dev], y_dev)
-        ms_step = timed(lambda: split([x_dev], y_dev), steps) / steps
+        ms_step = timed(keep(lambda: split([x_dev], y_dev)), steps) / steps
     elif graphed is not None:
         graphed.replay()
-        ms_step = timed(graphed.replay, steps) / steps
+        ms_step = timed(keep(graphed.replay), steps) / steps
     else:
         ms_step = eager_ms_step
     value = B * world / (ms_step / 1e3)
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, model_name, last['loss'], model)
 
     def e2e_loop(k):
         host_batches = ({'image': x_host, 'label': y_host} for _ in range(k))
@@ -637,6 +622,30 @@ def measure_model(model_name, args, rank, world, local_rank, dump_path=None, wit
     return rec
 
 
+DUMP_PARAMS = 1 << 21       # parameters kept per model by --dump-outputs (8 MB in float32)
+DUMP_LIMIT = 64 << 20
+
+
+def dump_outputs(out_dir, model_name, loss, model):
+    """What the last timed step hands its caller: the loss, and the model it trained - the parameters after the
+    optimizer step (all of them when there are at most DUMP_PARAMS, else DUMP_PARAMS at positions drawn with a fixed
+    seed from the concatenated parameter vector) and, for a model that has them, the floating-point buffers (BatchNorm
+    running statistics).  A model without such buffers (ViT) gets no buffers file rather than an empty one."""
+    os.makedirs(out_dir, exist_ok=True)
+    params = torch.cat([p.detach().float().reshape(-1) for p in model.parameters()])
+    if params.numel() > DUMP_PARAMS:
+        idx = torch.randperm(params.numel(), generator=torch.Generator().manual_seed(0))[:DUMP_PARAMS].sort().values
+        params = params[idx.to(params.device)]
+    bufs = [b.detach().double().reshape(-1) for b in model.buffers() if b.is_floating_point()]
+    arrays = {'loss': torch.as_tensor(loss).detach().float().reshape(1), 'params': params}
+    if bufs:
+        arrays['buffers'] = torch.cat(bufs)
+    for name, t in arrays.items():
+        np.save(os.path.join(out_dir, f'{model_name}_{name}.npy'), t.cpu().numpy())
+    total = sum(os.path.getsize(os.path.join(out_dir, f)) for f in os.listdir(out_dir) if f.endswith('.npy'))
+    assert total <= DUMP_LIMIT, f'--dump-outputs wrote {total} bytes (limit {DUMP_LIMIT})'
+
+
 def run_b200(args, rank, world, local_rank):
     dev = torch.device('cuda', local_rank)
     torch.cuda.set_device(dev)
@@ -663,7 +672,7 @@ def run_b200(args, rank, world, local_rank):
         return
     cpu_base = None
     if world == 1 and not args.no_cpu_baseline:
-        cpu_base = cpu_baseline_record(args.model, 16, 2, 5)
+        cpu_base = cpu_baseline_record(args.model, 16, 2, args.steps)
     line = {
         'metric': main['metric'], 'value': main['value'], 'unit': 'images/s', 'n_gpus': world, 'steps': args.steps,
         'warmup': max(3, args.warmup), 'ms_per_step': main['ms_per_step'], 'higher_is_better': True, 'scaling': 'weak',
@@ -712,6 +721,8 @@ def main():
     ap.add_argument('--model', default='resnet50', choices=['resnet50', 'vit_base_patch16'],
                     help='resnet50 = BASELINE configs[1] (default, the headline); vit_base_patch16 = configs[2]')
     ap.add_argument('--dump-ops', default=None, help='write the per-op timing table (csv) here')
+    ap.add_argument('--dump-outputs', default=None, metavar='DIR',
+                    help='after the timed steps, write what the last one computed (loss, trained parameters, buffers) as DIR/<model>_<name>.npy')
     ap.add_argument('--no-cpu-baseline', action='store_true')
     ap.add_argument('--no-second-model', action='store_true', help='skip the sub-record of the other BASELINE model')
     ap.add_argument('--detr', action='store_true', help='add the DETR-R50 sub-record (BASELINE configs[4]; shipped 1024x1024 shape, bs4)')

@@ -13,8 +13,8 @@ needed at run time), citing reference file:line for each function.
 
 Pinning: the reference has no tests or golden vectors (SURVEY.md §4).  The oracle is pinned
 against outputs of the reference itself: ``tests/golden/make_golden.py`` imports the reference
-from /root/reference in the build container and writes small fixtures (inputs, logits, loss,
-gradient digests) that ``tests/test_oracle_golden.py`` replays anywhere, and
-``tests/test_oracle_vs_reference.py`` compares oracle and reference live when /root/reference is
-present.
+(copied into oracle/_ref by oracle/install_ref.sh) and writes small fixtures (inputs, logits, loss,
+gradient digests) that ``tests/test_oracle_golden.py`` replays anywhere;
+``tests/golden/make_reference_snapshots.py`` does the same for ``tests/test_oracle_vs_reference.py``
+and the other tests that compare with the reference.
 """

@@ -13,7 +13,7 @@ for r in recs:
     summary.setdefault(r['model'], {})[f"{r['variant']}_n{r['n_gpus']}"] = {
         'images_per_sec': round(r['images_per_sec'], 1), 'ms_per_step': round(r['ms_per_step'], 2), 'amp_type': r['amp_type'],
         'per_gpu_batch': r['per_gpu_batch']}
-out = {'what': ("Unmodified reference modules (baseline/_ref install of /root/reference) driven by the reference's own tools/scripts.py "
+out = {'what': ("Unmodified reference modules (oracle/_ref copy of the reference) driven by the reference's own tools/scripts.py "
                 'train_classification loop under torch DistributedDataParallel + autocast on the same B200 pool '
                 '(baseline/torch_gpu_baseline.py).  Variants: as_shipped = fp16 autocast + GradScaler with cudnn.deterministic (the shipped '
                 'config; get_amp_type has no B200 entry); bf16 = the same loop with the amp whitelist forced to bfloat16; tuned = bf16 + '

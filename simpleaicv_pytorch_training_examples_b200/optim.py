@@ -6,7 +6,7 @@ separate cast / re-layout kernels: 53 per ResNet-50 step, 49 per ViT-B step) and
 without a host sync.  They subclass ``torch.optim.Optimizer``: ``param_groups`` (what ``tools.utils.Scheduler`` rewrites
 every iteration), ``state_dict()`` / ``load_state_dict()`` use torch's own keys (``momentum_buffer``; ``step``,
 ``exp_avg``, ``exp_avg_sq``), so checkpoints interchange with the reference's torch.optim.SGD / AdamW
-(/root/reference/tools/utils.py:581-600).
+(reference tools/utils.py:581-600).
 
 Hyper-parameters travel through a pinned ring of RING tables copied to the device at the head of every step; the kernel
 picks table (device step counter % RING).  Under CUDA-graph capture that copy is a node of the graph, so

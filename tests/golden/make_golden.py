@@ -1,5 +1,5 @@
-"""Generates tests/golden/*.pt by running the REFERENCE itself (imported from /root/reference, or
-from the baseline/_ref install) in the build container.  The fixtures are small: the seeded input
+"""Generates tests/golden/*.pt by running the REFERENCE itself (imported from the
+oracle/_ref copy, see baseline/ref_import.py).  The fixtures are small: the seeded input
 batch (or just its seed + a digest for the larger inputs), the logits / feature digest, the loss and
 per-parameter gradient digests (L2 norm + first 4 values); the weights are not stored because the
 oracle reproduces the reference's seeded initialisation exactly (checked here, bit for bit).
@@ -14,7 +14,12 @@ import torch
 HERE = os.path.dirname(os.path.abspath(__file__))
 ROOT = os.path.dirname(os.path.dirname(HERE))
 sys.path.insert(0, ROOT)
+sys.path.insert(0, HERE)
 from baseline import ref_import  # noqa: E402
+from make_reference_snapshots import take  # noqa: E402
+
+SAMPLED_NUMEL = 65536      # outputs larger than this are stored at SAMPLE_K fixed positions plus their L2 norm (files < 1 MB)
+SAMPLE_K = 8192
 
 # (tag, family, arch, kwargs, num_classes, batch shape, seed, store_x)
 CASES = [
@@ -36,7 +41,7 @@ CASES = [
       'window_size': 14, 'global_attn_indexes': (1,)}, 0, (1, 3, 320, 320), 8, False),
     # DETR (detection/models/detr.py): 6 + 6 transformer layers, 100 queries, padded right / bottom borders so that the
     # additive key-padding bias matters; dropout set to 0 on the reference; outputs = (cls, reg), loss = oracle.detr.surrogate_loss
-    ('resnet18_detr_b2_128x160', 'detr', 'resnet18_detr', {}, 80, (2, 3, 128, 160), 3, True),
+    ('resnet18_detr_b2_128x160', 'detr', 'resnet18_detr', {}, 80, (2, 3, 128, 160), 3, False),
 ]
 
 
@@ -204,6 +209,12 @@ def main():
                 fix['eval_logits'], fix['eval_reg'] = [t.clone() for t in model(x, detr_masks(shape))]
             else:
                 fix['eval_logits'] = model(x).clone()
+        if family == 'sam':
+            del fix['y']           # regenerated from the seed (sam_proj)
+        for k in ('logits', 'eval_logits'):
+            if fix[k].numel() > SAMPLED_NUMEL:
+                fix.setdefault('sampled', {})[k] = (SAMPLE_K, fix[k].double().norm().item())
+                fix[k] = take(fix[k], SAMPLE_K)
         torch.save(fix, os.path.join(HERE, tag + '.pt'))
         print(tag, 'loss', float(loss), os.path.getsize(os.path.join(HERE, tag + '.pt')), 'bytes')
 

@@ -1,5 +1,5 @@
 """Generates tests/golden/mae_b2_64px.ptm by running the REFERENCE's VITMAEPretrainModel + MSELoss
-(SimpleAICV/masked_image_modeling/models/vit_mae.py, losses.py; imported from /root/reference or baseline/_ref) on a small
+(SimpleAICV/masked_image_modeling/models/vit_mae.py, losses.py; imported from the oracle/_ref copy) on a small
 seeded case: ViT-B encoder width / decoder width 512 with 2 + 2 blocks, 64 px images (16 patches, 4 kept).  The masking
 noise is drawn once here and injected by replacing torch.rand for the duration of the reference forward, so that the
 reference's own random_masking code runs on known draws.  Stored: input, noise, prediction, mask, loss, gradient digests.

@@ -1,19 +1,30 @@
 """DETRLoss (detection/losses.py) against the committed reference outputs (tests/golden/detr_loss_b3.ptl, written by
-tests/golden/make_detr_loss_golden.py from the reference's DETRLoss) and, where the reference is installed, live.
-The Hungarian indices are integer work: they must match exactly."""
+tests/golden/make_detr_loss_golden.py from the reference's DETRLoss) and the reference's loss values on further
+inputs (tests/golden/reference_snapshots.pts).  The Hungarian indices are integer work: they must match exactly."""
 import importlib.util
 import os
 
 import pytest
 import torch
 
-from baseline import ref_import
 from simpleaicv_pytorch_training_examples_b200.detection.losses import DETRLoss, assignment_with_inf
 
 HERE = os.path.dirname(os.path.abspath(__file__))
 _spec = importlib.util.spec_from_file_location('mk', os.path.join(HERE, 'golden', 'make_detr_loss_golden.py'))
 mk = importlib.util.module_from_spec(_spec)
 _spec.loader.exec_module(mk)
+_spec = importlib.util.spec_from_file_location('make_reference_snapshots', os.path.join(HERE, 'golden', 'make_reference_snapshots.py'))
+snap = importlib.util.module_from_spec(_spec)
+_spec.loader.exec_module(snap)
+
+
+@pytest.fixture(autouse=True)
+def _one_thread():
+    """The reference snapshots were taken with one CPU thread: the same reduction order makes bit equality meaningful."""
+    n = torch.get_num_threads()
+    torch.set_num_threads(1)
+    yield
+    torch.set_num_threads(n)
 
 
 def test_detr_loss_reproduces_reference_fixture():
@@ -35,12 +46,11 @@ def test_detr_loss_reproduces_reference_fixture():
     torch.testing.assert_close(cls.grad.flatten()[:8], fix['dcls_head'], rtol=1e-5, atol=1e-8)
 
 
-@pytest.mark.skipif(not ref_import.available(), reason='reference not installed')
-@pytest.mark.parametrize('counts', [(1,), (2, 5, 1, 9), (100, 3)])
+@pytest.mark.parametrize('counts', snap.DETR_LOSS_COUNTS)
 def test_detr_loss_matches_reference_live(counts):
-    ref = ref_import.module('SimpleAICV.detection.losses').DETRLoss()
+    b = snap.load()[f'detr_loss/{counts}']
     cls, reg, ann = mk.make_inputs(seed=len(counts), counts=counts)
-    a, b = DETRLoss()([cls, reg], ann), ref([cls, reg], ann)
+    a = DETRLoss()([cls, reg], ann)
     assert list(a) == list(b) and all(torch.equal(a[k], b[k]) for k in b)
 
 

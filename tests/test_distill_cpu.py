@@ -1,38 +1,37 @@
 """Knowledge-distillation pieces (SURVEY.md 8 f4): the loss tails equal the reference's
-(SimpleAICV/distillation/losses.py) on the same logits, values and gradients; KDModel has the reference's layout."""
+(SimpleAICV/distillation/losses.py, its values and gradients on the same logits stored in
+tests/golden/reference_snapshots.pts); KDModel has the reference's layout."""
+import importlib.util
+import os
+
 import pytest
 import torch
 
-
-def _ref_losses():
-    from baseline import ref_import
-    if not ref_import.available():
-        pytest.skip('reference not present (GPU box)')
-    ref_import._ensure_path()
-    from SimpleAICV.distillation import losses
-    return losses
+HERE = os.path.dirname(os.path.abspath(__file__))
+_spec = importlib.util.spec_from_file_location('make_reference_snapshots', os.path.join(HERE, 'golden', 'make_reference_snapshots.py'))
+snap = importlib.util.module_from_spec(_spec)
+_spec.loader.exec_module(snap)
 
 
-@pytest.mark.parametrize('name,args', [('KDLoss', (4.0,)), ('DMLLoss', (2.0,)), ('L2Loss', ()), ('CELoss', ()), ('OneHotLabelCELoss', ())])
+@pytest.fixture(autouse=True)
+def _one_thread():
+    """The reference snapshots were taken with one CPU thread: the same reduction order makes bit equality meaningful."""
+    n = torch.get_num_threads()
+    torch.set_num_threads(1)
+    yield
+    torch.set_num_threads(n)
+
+
+@pytest.mark.parametrize('name,args', snap.DISTILL)
 def test_distillation_losses_match_reference(name, args):
-    ref = _ref_losses()
     from simpleaicv_pytorch_training_examples_b200.distillation import losses
-    g = torch.Generator().manual_seed(0)
-    stu = (torch.randn(16, 100, generator=g) * 3).requires_grad_(True)
-    stu2 = stu.detach().clone().requires_grad_(True)
-    tea = torch.randn(16, 100, generator=g) * 3
-    if name == 'CELoss':
-        other = torch.randint(0, 100, (16,), generator=g)
-    elif name == 'OneHotLabelCELoss':
-        other = torch.softmax(torch.randn(16, 100, generator=g), dim=1)
-    else:
-        other = tea
-    a = getattr(ref, name)(*args)(stu, other)
+    ref = snap.load()[f'distill/{name}']
+    stu2, other = snap.distill_inputs(name)
+    stu2.requires_grad_(True)
     b = getattr(losses, name)(*args)(stu2, other)
-    a.backward()
     b.backward()
-    assert torch.equal(a.detach(), b.detach())
-    assert torch.equal(stu.grad, stu2.grad)
+    assert torch.equal(ref['loss'], b.detach())
+    assert torch.equal(ref['grad'], stu2.grad)
 
 
 def test_kdmodel_layout_and_frozen_teacher():

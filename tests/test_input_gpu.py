@@ -1,6 +1,6 @@
 """Input-pipeline edge (SURVEY.md 8 f3): uint8 batches normalised on the device are BIT-identical to the reference's host
 pipeline - TorchMeanStdNormalize (ToTensor: uint8 HWC -> float CHW / 255; Normalize: sub_(mean).div_(std);
-/root/reference/SimpleAICV/classification/common.py:228-248) followed by ClassificationCollater's stack + permute
+reference SimpleAICV/classification/common.py:228-248) followed by ClassificationCollater's stack + permute
 (:645-665) - for vector-friendly and odd image sizes, directly and through the prefetcher."""
 import numpy as np
 import pytest

@@ -1,6 +1,6 @@
 """MAE pre-training (SURVEY.md 8 f4): the oracle (oracle/mae.py) replays outputs of the REFERENCE's VITMAEPretrainModel +
-MSELoss (tests/golden/mae_b2_64px.ptm, made by tests/golden/make_mae_golden.py), matches the live reference when it is
-present, and the B200 module shell has the reference's state_dict and seeded initialisation.  CPU only."""
+MSELoss (tests/golden/mae_b2_64px.ptm, made by tests/golden/make_mae_golden.py), matches the reference's state dict and
+gradients (tests/golden/reference_snapshots.pts), and the B200 module shell has the reference's state_dict and seeded initialisation.  CPU only."""
 import importlib.util
 import os
 
@@ -13,6 +13,9 @@ ARCH = 'vit_base_patch16_224_mae_pretrain_model'
 _spec = importlib.util.spec_from_file_location('make_mae_golden', os.path.join(HERE, 'golden', 'make_mae_golden.py'))
 gen = importlib.util.module_from_spec(_spec)
 _spec.loader.exec_module(gen)
+_spec = importlib.util.spec_from_file_location('make_reference_snapshots', os.path.join(HERE, 'golden', 'make_reference_snapshots.py'))
+snap = importlib.util.module_from_spec(_spec)
+_spec.loader.exec_module(snap)
 
 
 def _fixture():
@@ -37,22 +40,17 @@ def test_oracle_reproduces_reference_mae_outputs():
 
 
 def test_oracle_matches_live_reference_mae():
-    from baseline import ref_import
-    if not ref_import.available():
-        pytest.skip('reference not present (GPU box)')
     from oracle import mae
+    ref = snap.load()['mae']
     torch.set_num_threads(1)
     x, noise = gen.make_inputs()
-    model, pred, mask, loss, grads = gen.reference_run(x, noise)
     sd = mae.init_state(ARCH, gen.SEED, image_size=gen.CFG['image_size'], enc_depth=2, dec_depth=2)
-    for k, v in model.state_dict().items():
-        assert torch.equal(v, sd[k]), k
+    snap.check_state(ref['state'], sd)
     opred, omask, oloss, ograds = mae.loss_and_grads(sd, x, noise, ARCH, enc_depth=2, dec_depth=2)
-    assert torch.equal(omask, mask)
-    torch.testing.assert_close(opred, pred, rtol=1e-5, atol=1e-5)
-    torch.testing.assert_close(oloss, loss, rtol=1e-5, atol=1e-6)
-    for n, g in grads.items():
-        torch.testing.assert_close(ograds[n], g, rtol=1e-4, atol=1e-6)
+    assert torch.equal(omask, ref['mask'])
+    snap.check_close(ref['pred'], {'pred': opred}, rtol=1e-5, atol=1e-5)
+    torch.testing.assert_close(oloss, ref['loss'], rtol=1e-5, atol=1e-6)
+    snap.check_close(ref['grads'], ograds, rtol=1e-4, atol=1e-6)
 
 
 @pytest.mark.parametrize('kw', [dict(image_size=64, enc=2, dec=2), dict(image_size=32, enc=1, dec=3)])

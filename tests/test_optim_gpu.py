@@ -1,5 +1,5 @@
 """Fused multi-tensor optimizers (optim.py, csrc/capi_optim.cu) against torch.optim.SGD / AdamW - the optimizers the
-reference builds (/root/reference/tools/utils.py:581-600) - on identical parameters and gradients: several steps with
+reference builds (reference tools/utils.py:581-600) - on identical parameters and gradients: several steps with
 per-group learning rates / weight decays that change every step, odd sizes and unaligned gradient views, the fused bf16
 operand copies (Linear and conv tap-major layouts), the fused global-norm clip, state_dict interchange and a captured
 step with a per-iteration learning rate."""

@@ -1,11 +1,10 @@
 """Host-side logic of the tools layer: optimizer parameter groups and LR schedule.
 
-Runs on CPU.  Where /root/reference exists the results are compared with the reference's own
-tools/utils.py (its `calflops` import is stubbed — the hot path never calls it)."""
+Runs on CPU.  The results are compared with what the reference's own tools/utils.py and classification/common.py
+give on the same models (stored in tests/golden/reference_snapshots.pts by tests/golden/make_reference_snapshots.py)."""
+import importlib.util
 import math
 import os
-import sys
-import types
 
 import pytest
 import torch
@@ -13,7 +12,10 @@ import torch
 from simpleaicv_pytorch_training_examples_b200.classification import backbones
 from simpleaicv_pytorch_training_examples_b200.tools import utils as my_utils
 
-REF = '/root/reference'
+HERE = os.path.dirname(os.path.abspath(__file__))
+_spec = importlib.util.spec_from_file_location('make_reference_snapshots', os.path.join(HERE, 'golden', 'make_reference_snapshots.py'))
+snap = importlib.util.module_from_spec(_spec)
+_spec.loader.exec_module(snap)
 
 
 class _Cfg:
@@ -56,57 +58,36 @@ def test_scheduler_closed_forms(name, params):
         assert abs(opt.param_groups[0]['lr'] - exp) < 1e-12 and abs(s.current_lr - exp) < 1e-12
 
 
-def _ref_utils():
-    from baseline import ref_import
-    if not ref_import.available():
-        pytest.skip('reference not installed (baseline/install_ref.sh)')
-    return ref_import.module('tools.utils')
-
-
-def _canon(o):
-    return sorted((g['weight_decay'], round(g['lr'], 15), sorted(id(p) for p in g['params'])) for g in o.param_groups)
+def _ref_tools():
+    return snap.load()['tools']
 
 
 def test_vit_layer_decay_groups_match_reference_utils():
     """ViT layer-wise lr decay + no-weight-decay name list (tools/utils.py:313-420), the AdamW setting of
     00.classification_training/imagenet/vit_base_patch16_*/train_config.py."""
-    ref_utils = _ref_utils()
+    ref = _ref_tools()['vit_layer_decay']
     m = backbones.vit_base_patch16(image_size=32, num_classes=10)
-
-    class C:
-        optimizer = ('AdamW', {'lr': 5e-4, 'global_weight_decay': False, 'weight_decay': 0.05,
-                               'no_weight_decay_layer_name_list': ['position_encoding', 'cls_token'],
-                               'lr_layer_decay': 0.65, 'lr_layer_decay_block': m.blocks, 'block_name': 'blocks'})
-        scheduler = ('CosineLR', {'warm_up_epochs': 5, 'min_lr': 1e-6})
-        epochs = 100
-    ro, _ = ref_utils.build_optimizer(C, m)
+    C = snap.vit_cfg(m)
     mo, _ = my_utils.build_optimizer(C, m)
-    assert _canon(ro) == _canon(mo)
-    assert type(ro) is type(mo) and ro.defaults['betas'] == mo.defaults['betas'] and ro.defaults['eps'] == mo.defaults['eps']
-    rs, ms = ref_utils.Scheduler(C, ro), my_utils.Scheduler(C, mo)
-    for e in [0.0, 2.5, 5.0, 50.0, 99.5]:
-        rs.step(ro, e)
+    assert ref['groups'] == snap.canon_groups(mo, m)
+    assert ref['type'] == type(mo).__name__ and ref['betas'] == mo.defaults['betas'] and ref['eps'] == mo.defaults['eps']
+    ms = my_utils.Scheduler(C, mo)
+    for e, lr, groups in zip(snap.VIT_EPOCHS, ref['lr'], ref['groups_after']):
         ms.step(mo, e)
-        assert abs(rs.current_lr - ms.current_lr) < 1e-15
-        assert _canon(ro) == _canon(mo)
+        assert abs(lr - ms.current_lr) < 1e-15
+        assert groups == snap.text_hash(snap.canon_groups(mo, m))
 
 
 def test_groups_and_schedule_match_reference_utils():
-    ref_utils = _ref_utils()
+    ref = _ref_tools()['r50_groups']
     m = backbones.resnet50cifar(num_classes=10)
-    ro, _ = ref_utils.build_optimizer(_Cfg, m)
-    mo, _ = my_utils.build_optimizer(_Cfg, m)
-
-    def canon(o):
-        return sorted((g['weight_decay'], g['lr'], sorted(id(p) for p in g['params'])) for g in o.param_groups)
-
-    assert canon(ro) == canon(mo)
-    rs, ms = ref_utils.Scheduler(_Cfg, ro), my_utils.Scheduler(_Cfg, mo)
-    for e in [0.0, 0.5, 0.99, 1.0, 29.9, 30.0, 61.2, 95.0]:
-        rs.step(ro, e)
+    mo, _ = my_utils.build_optimizer(snap.R50Cfg, m)
+    assert ref['groups'] == snap.canon_groups(mo, m)
+    ms = my_utils.Scheduler(snap.R50Cfg, mo)
+    for e, lr, group_lrs in zip(snap.R50_EPOCHS, ref['lr'], ref['group_lrs']):
         ms.step(mo, e)
-        assert abs(rs.current_lr - ms.current_lr) < 1e-12
-        assert sorted(g['lr'] for g in ro.param_groups) == sorted(g['lr'] for g in mo.param_groups)
+        assert abs(lr - ms.current_lr) < 1e-12
+        assert group_lrs == sorted(g['lr'] for g in mo.param_groups)
 
 
 def test_checkpoint_key_layout_matches_reference_and_round_trips():
@@ -144,25 +125,17 @@ def test_meters_and_amp_type_match_reference():
     returns bf16 for CPU-resident models (no device to inspect) and has 'B200' in its whitelist."""
     import inspect
     import torch
-    from baseline import ref_import
     from simpleaicv_pytorch_training_examples_b200.classification import common
-    if ref_import.available():
-        rc = ref_import.module('SimpleAICV.classification.common')
-        pairs = [(common.AverageMeter(), rc.AverageMeter()), (common.AccMeter(), rc.AccMeter())]
-    else:
-        pairs = [(common.AverageMeter(), None), (common.AccMeter(), None)]
-    a, ra = pairs[0]
+    ref = _ref_tools()['meters']
+    a = common.AverageMeter()
     for v, n in [(1.5, 4), (0.25, 2), (3.0, 1)]:
         a.update(v, n)
-        ra.update(v, n) if ra is not None else None
-    assert abs(a.avg - (1.5 * 4 + 0.5 + 3.0) / 7) < 1e-12 and (ra is None or (a.avg, a.sum, a.count, a.val) == (ra.avg, ra.sum, ra.count, ra.val))
-    m, rm = pairs[1]
+    assert abs(a.avg - (1.5 * 4 + 0.5 + 3.0) / 7) < 1e-12 and (a.avg, a.sum, a.count, a.val) == ref['average']
+    m = common.AccMeter()
     for c1, c5, n in [(3, 7, 10), (5, 9, 10)]:
         m.update(c1, c5, n)
-        rm.update(c1, c5, n) if rm is not None else None
     m.compute()
-    rm.compute() if rm is not None else None
-    assert (m.acc1, m.acc5) == (0.4, 0.8) and (rm is None or (m.acc1, m.acc5) == (rm.acc1, rm.acc5))
+    assert (m.acc1, m.acc5) == (0.4, 0.8) and (m.acc1, m.acc5) == ref['acc']
     assert "'B200'" in inspect.getsource(common.get_amp_type)
     assert common.get_amp_type(torch.nn.Linear(2, 2)) == torch.bfloat16
 
